@@ -24,6 +24,10 @@ One JSON line on rank 0:
   cpu_baseline  the oracle port (CPU restatement of the reference, oracle/cotr_oracle.py) on the host cores, rank 0, N=1
 `--impl reference` times that CPU path alone (all host threads) and prints the same line shape with "impl": "reference".
 `--config 3` / `--config 5` time the zoom-in engines instead (see DESIGN.md section 6).
+`--dump-outputs DIR` writes what the last timed step returned to its caller as DIR/<name>.npy (float32): `pred_corrs`
+(1,1024,2) of rank 0, and for N > 1 `pred_corrs_gathered` (N,1024,2), the block the result exchange delivered.  Weights
+and inputs are seeded, so runs with the same arguments see the same inputs and two builds can be compared output for
+output.
 """
 import argparse
 import json
@@ -238,8 +242,10 @@ def run_reference(args, rank, world):
         cotr_oracle.forward(sd, img, queries, torch.float32)
     for _ in range(args.steps):
         t0 = time.perf_counter()
-        cotr_oracle.forward(sd, img, queries, torch.float32)
+        pred = cotr_oracle.forward(sd, img, queries, torch.float32)
         steps.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"pred_corrs": pred})
     # the host is shared and noisy (round 1: 8.3-9.9 k q/s across records): the median step is the robust figure
     ms = float(np.median(steps)) * 1e3
     value = N_QUERIES / (ms * 1e-3)
@@ -253,6 +259,15 @@ def run_reference(args, rank, world):
         "dtype": "f32", "data": "synthetic", "config": config_dict(args.gpus),
         "cpu_baseline": base, "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0}))
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: every array (torch tensor or numpy) as out_dir/<name>.npy in float32."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if not isinstance(a, np.ndarray):
+            a = a.detach().cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
 
 
 def _timed_steps(step, flush, n, barrier):
@@ -335,6 +350,11 @@ def run_native(args, rank, local_rank, world):
         per_rank[rank, 0], per_rank[rank, 1] = dev_ms, solo_ms
         dist.all_reduce(per_rank)
         rank_ms = per_rank.tolist()
+    if args.dump_outputs and rank == 0:
+        outputs = {"pred_corrs": last["pred"]}
+        if world > 1:
+            outputs["pred_corrs_gathered"] = got
+        dump_outputs(args.dump_outputs, outputs)
 
     # ---- e2e: host buffers in, host result out, every copy inside the timed region ----------------------------------
     img_h, q_h, out_h = img_pin.numpy(), q_pin.numpy(), out_pin.numpy()
@@ -484,14 +504,20 @@ def run_native(args, rank, local_rank, world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=50, help="timed steps (at least 1)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", choices=["native", "reference"], default="native")
     ap.add_argument("--quick", action="store_true",
                     help="headline steps only (no configs[3] block, no CPU baseline, no clock continuation): the form to run under ncu")
     ap.add_argument("--config", type=int, default=2, choices=[2, 3, 5],
                     help="2 = the headline (default); 3 / 5 = the zoom-in engines of BASELINE.json configs[2] / configs[4]")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (float32); headline config only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.config != 2:
+        ap.error("--dump-outputs is available for the headline config (--config 2) only")
     if args.gpus > 1 and "WORLD_SIZE" not in os.environ:
         # `python bench.py --gpus N` without a launcher: become `torch.distributed.run` with N ranks on this node
         os.execvp(sys.executable, [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={args.gpus}",

@@ -30,10 +30,14 @@ CASES = {
     "model_b64_q1024": (0, 3.0, 1.35, 7, 64, 1024, 1.0, 16),     # BASELINE.json configs[3] (64 pairs x 1024 queries)
     "model_bigact_b1_q256": (0, 3.0, 1.35, 8, 1, 256, 160.0, 1),  # backbone activations up to ~4e4 (fp16 hi/lo range)
 }
+# The fp32 round-off of a CPU forward depends on torch's intra-op thread count (model_b1_q1024 moves by 9e-5 at 1
+# thread and by 5e-5 at 16 or more against 4 or 8), so the fp32 vectors are recorded, and checked, with this many.
+GOLDEN_THREADS = 8
 
 
 def main():
     torch.set_grad_enabled(False)
+    torch.set_num_threads(GOLDEN_THREADS)
     out_dir = os.path.join(REPO, "tests", "golden")
     os.makedirs(out_dir, exist_ok=True)
     only = sys.argv[1:]

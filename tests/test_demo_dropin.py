@@ -1,147 +1,128 @@
-"""BASELINE.json configs[0]: the reference's own `demo_single_pair.py` executed UNMODIFIED against this repository.
+"""BASELINE.json configs[0]: the reference's `demo_single_pair.py` against this repository, held to what the reference
+itself did with the same inputs.
 
-The script's imports (`from COTR.models import build_model`, `from COTR.inference.sparse_engine import SparseEngine`,
-`from COTR.options.options import *` ...) bind to the alias package `COTR/` -> `cotr_b200`; what it needs from outside
-the hot path is injected exactly as SURVEY.md section 8(d) spells out: stand-ins for the two packages that are not
-installed offline (`imageio`, `matplotlib`), a synthetic `out/default/checkpoint.pth.tar` in the reference's checkpoint
-format (`{'model_state_dict': ...}` with the 381-entry schema, loaded by `utils.safe_load_weights` with strict=True) and the
-reference's `sample_data/` images.  With seeded synthetic weights the network's answers are not meaningful, so
+tests/golden/demo_single_pair.npz was made by running that script, unmodified, against the reference's own package
+(oracle/make_demo_golden.py) on seeded synthetic stand-ins for the sample pair and a seeded synthetic checkpoint.
+`_demo_main` below makes the script's calls in the script's order, but through the alias package `COTR/` -> `cotr_b200`
+(`from COTR.models import build_model`, `from COTR.inference.sparse_engine import SparseEngine`, `from
+COTR.options.options import *` ...), with the same inputs:
 
-  * the CPU test (no GPU needed) puts the deterministic stand-in network of `oracle/fake_model.py` behind
-    `build_model` - same parameter schema, same `model(img, queries)['pred_corrs']` contract - and checks that the whole
-    script (model construction, strict checkpoint load, SparseEngine cycle-consistent matching, visualisation,
-    `triangulate_corr`, the final `cv2.remap`) runs to its last line and produces `--max_corrs` correspondences;
-  * the GPU test runs the real native model through the same script; random weights accept no task (SURVEY.md section
-    8c: the reference itself dies on `assert corr_f.shape[0] > 0`, sparse_engine.py:247), so it asserts exactly that
-    documented outcome after the dense passes and the zoom-in batches have run on the device.
-Both are skipped where `/root/reference` does not exist (the GPU box): nothing here reads it at import time.
+  * the CPU test puts the deterministic stand-in network of `oracle/fake_model.py` behind `build_model` - same
+    parameter schema (so the strict checkpoint load is the real one), same `model(img, queries)['pred_corrs']`
+    contract - and demands the reference's network calls, correspondences and final blended image;
+  * the GPU test runs the real native model; seeded random weights accept no task, and the reference ends in
+    `assert corr_f.shape[0] > 0` (sparse_engine.py:247, SURVEY.md section 8c).  The native run must end there too,
+    after the dense passes and the zoom-in batches have run on the device.
 """
+import argparse
 import os
-import runpy
 import sys
-import types
+import traceback
 
 import numpy as np
 import pytest
 import torch
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
-DEMO = os.path.join(REF, "demo_single_pair.py")
-
-needs_reference = pytest.mark.skipif(not os.path.exists(DEMO), reason="the reference tree is not present on this machine")
 
 
-def _stand_ins(monkeypatch, shown):
-    """`imageio.imread(path, pilmode='RGB')` and `matplotlib.pyplot.imshow/show` (not installed offline)."""
+def _golden(golden_dir):
+    return np.load(os.path.join(golden_dir, "demo_single_pair.npz"))
+
+
+def _demo_main(tmp_path, max_corrs, prepare_model=None, triangulate=None):
+    """What demo_single_pair.py does between its imports and plt.show(), through the `COTR` alias package.
+    Returns (model, corrs, blended image)."""
     import cv2
-    imageio = types.ModuleType("imageio")
-    imageio.imread = lambda path, pilmode="RGB": cv2.cvtColor(cv2.imread(path, cv2.IMREAD_COLOR), cv2.COLOR_BGR2RGB)
-    mpl = types.ModuleType("matplotlib")
-    plt = types.ModuleType("matplotlib.pyplot")
-    plt.imshow = lambda img, *a, **k: shown.append(np.asarray(img))
-    plt.show = lambda *a, **k: None
-    mpl.pyplot = plt
-    monkeypatch.setitem(sys.modules, "imageio", imageio)
-    monkeypatch.setitem(sys.modules, "matplotlib", mpl)
-    monkeypatch.setitem(sys.modules, "matplotlib.pyplot", plt)
-
-
-def _workdir(tmp_path, monkeypatch, max_corrs):
+    sys.path.insert(0, REPO)
+    from COTR.inference import inference_helper
+    from COTR.inference.sparse_engine import SparseEngine
+    from COTR.models import build_model
+    from COTR.options.options import set_COTR_arguments
+    from COTR.utils import utils
     from cotr_b200.utils import synthetic
-    os.symlink(os.path.join(REF, "sample_data"), tmp_path / "sample_data")
-    ckpt_dir = tmp_path / "out" / "default"
-    ckpt_dir.mkdir(parents=True)
+    from oracle.make_demo_golden import demo_image
+
+    ckpt = tmp_path / "out" / "default" / "checkpoint.pth.tar"
+    ckpt.parent.mkdir(parents=True)
     sd = {k: torch.from_numpy(v) for k, v in synthetic.make_state_dict(0).items()}
-    torch.save({"epoch": 0, "iteration": 0, "optim_state_dict": {}, "model_state_dict": sd}, ckpt_dir / "checkpoint.pth.tar")
-    monkeypatch.chdir(tmp_path)
-    monkeypatch.syspath_prepend(REPO)
-    monkeypatch.setattr(sys, "argv", ["demo_single_pair.py", "--load_weights", "default", "--max_corrs", str(max_corrs),
-                                      "--out_dir", str(tmp_path / "out")])
+    torch.save({"epoch": 0, "iteration": 0, "optim_state_dict": {}, "model_state_dict": sd}, ckpt)
+    parser = argparse.ArgumentParser()
+    set_COTR_arguments(parser)
+    opt = parser.parse_args([])
+    opt.dim_feedforward = 1024                         # layer3
+    utils.fix_randomness(0)
+    with torch.set_grad_enabled(False):
+        model = build_model(opt)
+        if prepare_model is not None:
+            prepare_model(model)
+        model = model.cuda()
+        utils.safe_load_weights(model, torch.load(ckpt, map_location='cpu')['model_state_dict'])
+        model = model.eval()
+        img_a, img_b = demo_image("cathedral_1.jpg"), demo_image("cathedral_2.jpg")
+        engine = SparseEngine(model, 32, mode='tile')
+        corrs = engine.cotr_corr_multiscale_with_cycle_consistency(img_a, img_b, np.linspace(0.5, 0.0625, 4), 1,
+                                                                   max_corrs=max_corrs, queries_a=None)
+        utils.visualize_corrs(img_a, img_b, corrs)
+        dense = (triangulate or inference_helper.triangulate_corr)(corrs, img_a.shape, img_b.shape)
+        warped = cv2.remap(img_b, dense[..., 0].astype(np.float32), dense[..., 1].astype(np.float32),
+                           interpolation=cv2.INTER_LINEAR, borderMode=cv2.BORDER_CONSTANT)
+        return model, corrs, warped / 255 * 0.5 + img_a / 255 * 0.5
 
 
-@needs_reference
-def test_demo_single_pair_runs_unmodified_cpu(tmp_path, monkeypatch, capsys):
-    import cotr_b200.models as models
-    from cotr_b200.inference import inference_helper
-    from cotr_b200.models.cotr_model import COTR
+def test_demo_single_pair_matches_reference_cpu(golden_dir, tmp_path, capsys):
     from oracle import triangulate_oracle
     from oracle.fake_model import FakeCOTR
+    from oracle.make_demo_golden import FAKE_MAX_CORRS, blend_summary
+    from oracle.make_engine_golden import call_log_array
+    gold = _golden(golden_dir)
 
-    class FakeBehindTheSchema(COTR):
-        """The real parameter tree (so the strict checkpoint load is the real one) around the stand-in arithmetic."""
-        supports_device_preprocess = False
+    def fake_network(model):
+        object.__setattr__(model, "fake", FakeCOTR())      # not a registered sub-module: the schema stays the reference's
+        model.forward = model.fake.forward
+        model.supports_device_preprocess = False
+        model.cuda = lambda *a, **k: model                 # no GPU needed: the stand-in runs on the host
 
-        def __init__(self, args=None):
-            super().__init__(args)
-            self.__dict__['fake'] = FakeCOTR()      # not a registered sub-module: the parameter schema stays the reference's
-            self.loaded = 0
-
-        def cuda(self, device=None):
-            return self
-
-        def load_state_dict(self, state_dict, *a, **k):
-            self.loaded += 1
-            return torch.nn.Module.load_state_dict(self, state_dict, *a, **k)
-
-        def forward(self, samples, queries):
-            return self.fake(samples, queries)
-
-    built = []
-
-    def fake_build_model(args):
-        built.append(FakeBehindTheSchema(args))
-        return built[-1]
-
-    shown = []
-    _stand_ins(monkeypatch, shown)
-    _workdir(tmp_path, monkeypatch, max_corrs=40)
-    monkeypatch.setattr(models, "build_model", fake_build_model)
-    # the product triangulate_corr renders with CUDA; this machine has no GPU, so the script gets the CPU restatement
-    monkeypatch.setattr(inference_helper, "triangulate_corr",
-                        lambda corr, a, b: triangulate_oracle.triangulate_corr(corr, a, b)[0])
-    runpy.run_path(DEMO, run_name="__main__")
-    out = capsys.readouterr().out
-    assert "weights safely loaded" in out                       # utils.safe_load_weights, strict path
-    assert "seconds for 40 correspondences" in out               # the script's own last report
-    assert built and built[0].loaded == 1 and len(built[0].fake.calls) > 8      # 4 dense passes + the zoom-in batches
-    assert built[0].fake.calls[0][1] == (1, 256 * 512, 2)        # cotr_flow's 131 072-query pass came first
-    assert len(shown) == 1 and shown[0].shape == (783, 1064, 3)  # warped image blended over cathedral_1.jpg
+    # the product triangulate_corr renders with CUDA; on the host the script gets the CPU restatement, as the reference did
+    model, corrs, shown = _demo_main(tmp_path, FAKE_MAX_CORRS, fake_network,
+                                     lambda corr, a, b: triangulate_oracle.triangulate_corr(corr, a, b)[0])
+    assert "weights safely loaded" in capsys.readouterr().out      # utils.safe_load_weights, strict path
+    calls = call_log_array(model.fake)
+    assert calls.shape == gold["fake_calls"].shape                 # 4 dense passes + the zoom-in batches
+    assert np.array_equal(calls[:, :2], gold["fake_calls"][:, :2])
+    np.testing.assert_allclose(calls[:, 2:], gold["fake_calls"][:, 2:], rtol=1e-12, atol=1e-9)
+    assert corrs.shape == (FAKE_MAX_CORRS, 4)
+    np.testing.assert_array_equal(corrs, gold["fake_corrs"])
+    got = blend_summary(shown)
+    np.testing.assert_array_equal(got["shown_shape"], gold["shown_shape"])        # warped image blended over image a
+    np.testing.assert_allclose(got["shown_sum"], gold["shown_sum"], rtol=1e-12)
+    np.testing.assert_allclose(got["shown_abs"], gold["shown_abs"], rtol=1e-12)
+    np.testing.assert_allclose(got["shown_sample"], gold["shown_sample"], rtol=1e-12, atol=1e-12)
 
 
-@needs_reference
 @pytest.mark.gpu
-def test_demo_single_pair_runs_unmodified_gpu(tmp_path, monkeypatch, capsys, built_lib):
-    """The same script, native model on the GPU, 100 correspondences requested (the demo's default).  Seeded random
-    weights are rejected by the engine's own acceptance tests, which the reference turns into
-    `assert corr_f.shape[0] > 0` (sparse_engine.py:247) - reproduced here as the expected end of the run."""
-    import cotr_b200.models as models
-    real_build = models.build_model
+def test_demo_single_pair_native_ends_like_reference_gpu(golden_dir, tmp_path, capsys, built_lib):
+    """The same calls, native model on the GPU, 100 correspondences requested (the demo's default).  Seeded random
+    weights are rejected by the engine's own acceptance tests: the run must end where the reference's ended."""
+    from oracle.make_demo_golden import NETWORK_MAX_CORRS, failure_site
+    gold = _golden(golden_dir)
     built = []
-
-    def build_and_keep(args):
-        built.append(real_build(args))
-        return built[-1]
-
-    shown = []
-    _stand_ins(monkeypatch, shown)
-    _workdir(tmp_path, monkeypatch, max_corrs=100)
-    monkeypatch.setattr(models, "build_model", build_and_keep)
-    with pytest.raises(AssertionError):
-        runpy.run_path(DEMO, run_name="__main__")
-    out = capsys.readouterr().out
-    assert "weights safely loaded" in out
+    with pytest.raises(AssertionError) as info:
+        _demo_main(tmp_path, NETWORK_MAX_CORRS, built.append)
+    assert failure_site(info.value) == (str(gold["network_failure_function"]), str(gold["network_failure_line"])), \
+        traceback.format_exception(info.value)
+    assert "weights safely loaded" in capsys.readouterr().out
     assert built and next(built[0].parameters()).is_cuda
     assert built[0].native().last_launch_count() > 50            # the device really ran the network
 
 
 @pytest.mark.gpu
 def test_demo_call_sequence_native_gpu(tmp_path, capsys, built_lib):
-    """What `demo_single_pair.py:25-45` does, restated for the GPU box (where the reference tree does not exist), with
-    the changes SURVEY.md section 8(d) prescribes for random weights: synthetic images instead of the sample pair and
-    100 FORCED queries (`cotr_corr_multiscale(..., queries_a=q, force=True)`), so every query comes back.  Everything
-    goes through the alias package `COTR`, as in the script: build_model -> cuda -> checkpoint file -> safe_load_weights ->
-    SparseEngine(model, 32, mode='tile') -> visualize_corrs -> triangulate_corr (CUDA rasteriser) -> cv2.remap."""
+    """What `demo_single_pair.py:25-45` does, with the changes SURVEY.md section 8(d) prescribes for random weights:
+    synthetic images instead of the sample pair and 100 FORCED queries (`cotr_corr_multiscale(..., queries_a=q,
+    force=True)`), so every query comes back.  Everything goes through the alias package `COTR`, as in the script:
+    build_model -> cuda -> checkpoint file -> safe_load_weights -> SparseEngine(model, 32, mode='tile') ->
+    visualize_corrs -> triangulate_corr (CUDA rasteriser) -> cv2.remap."""
     import cv2
     sys.path.insert(0, REPO)
     from COTR.utils import utils

@@ -7,6 +7,7 @@ import pytest
 import torch
 
 from oracle import cotr_oracle, fixtures
+from oracle.make_golden import GOLDEN_THREADS
 
 CASES = sorted(os.path.basename(p)[:-4] for p in glob.glob(os.path.join(os.path.dirname(__file__), "golden", "model_*.npz")))
 
@@ -25,8 +26,17 @@ def test_golden_files_exist():
     assert len(CASES) >= 4
 
 
+@pytest.fixture
+def golden_threads():
+    """The intra-op thread count the fp32 goldens were recorded with (their round-off depends on it)."""
+    n = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(n)
+
+
 @pytest.mark.parametrize("name", CASES)
-def test_oracle_fp32_matches_reference_fp32(golden_dir, name):
+def test_oracle_fp32_matches_reference_fp32(golden_dir, golden_threads, name):
     g, sd, img, queries, q_stride = _load(golden_dir, name)
     pred = cotr_oracle.forward(sd, img, queries, torch.float32).numpy()[:, ::q_stride]
     # same arithmetic, same library kernels: the restatement reproduces the reference to fp32 round-off
