@@ -65,6 +65,7 @@ _PROTOTYPES = {
     "cotr_profile_end": (ctypes.c_int, [ctypes.c_void_p, ctypes.POINTER(LaunchRecord), ctypes.c_int]),
     "cotr_debug_read": (ctypes.c_int64, [ctypes.c_void_p, ctypes.c_char_p, ctypes.c_void_p, ctypes.c_int64]),
     "cotr_set_gemm_path": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int]),
+    "cotr_set_batch_invariant": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int]),
     "cotr_test_gemm": (ctypes.c_int, [ctypes.POINTER(TestGemmDesc)] + [ctypes.c_void_p] * 9),
     "cotr_test_attention": (ctypes.c_int, [ctypes.c_int] + [ctypes.c_void_p] * 4 + [ctypes.c_int, ctypes.c_int]),
     "cotr_debug_set_variant": (None, [ctypes.c_int]),
@@ -220,6 +221,10 @@ class NativeModel:
 
     def set_gemm_path(self, path):
         check(lib().cotr_set_gemm_path(self.handle, int(path)), "cotr_set_gemm_path")
+
+    def set_batch_invariant(self, enabled):
+        """Batch-invariant mode (cotr_set_batch_invariant): the headline schedule for every pair and query."""
+        check(lib().cotr_set_batch_invariant(self.handle, int(bool(enabled))), "cotr_set_batch_invariant")
 
     def last_launch_count(self):
         return lib().cotr_last_launch_count(self.handle)

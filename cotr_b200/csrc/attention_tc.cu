@@ -60,6 +60,12 @@ __device__ __forceinline__ float fast_exp2(float x) {
     return y;
 }
 
+// kSkipIdle (launches with nq < 32 only): softmax warps whose 32-row TMEM lane quarter holds no valid query row skip the
+// TMEM reads, the exponentials and the P stores; they still wait on and arrive at every barrier like the others, so the
+// arrival counts are unchanged.  The MMA then multiplies stale P rows of those lanes, whose output rows are never read.
+// The rows of the other quarters run exactly the instructions of the default instantiation.  A separate instantiation
+// because a flag-guarded path that never executes still slows a tcgen05 kernel down (DESIGN.md section 8).
+template <bool kSkipIdle>
 __global__ void __launch_bounds__(kThreads, 1) attention_tc_kernel(const AttnParams p, long long* __restrict__ ts) {
     // debug timeline (ts != null, cotr_debug_set_timestamps): 64 clock64() stamps per CTA, slots in tools/bringup.py
     long long* my_ts = ts ? ts + (size_t)((blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x) * 64 : nullptr;
@@ -113,6 +119,7 @@ __global__ void __launch_bounds__(kThreads, 1) attention_tc_kernel(const AttnPar
         const int trow_i = quarter * 32 + lane;          // query row inside the tile == TMEM lane
         const int qi = row0 + trow_i;
         const bool row_ok = qi < p.nq;
+        const bool idle = kSkipIdle && row0 + quarter * 32 >= p.nq;      // warp-uniform: no valid row in this lane quarter
         const size_t grow = (size_t)pair_local * p.nq + (row_ok ? qi : 0);
         const size_t kv_row0 = (size_t)(p.pair0 + pair_local) * kTokens;
         if (t == 0) {
@@ -186,7 +193,7 @@ __global__ void __launch_bounds__(kThreads, 1) attention_tc_kernel(const AttnPar
         const uint32_t trow = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(half * 32);
         float mx = -INFINITY;
 #pragma unroll 1
-        for (int c = 0; c < kTokens; c += 128) {
+        for (int c = 0; c < (idle ? 0 : kTokens); c += 128) {
             uint32_t r[4][16];
             __syncwarp();
 #pragma unroll
@@ -198,10 +205,12 @@ __global__ void __launch_bounds__(kThreads, 1) attention_tc_kernel(const AttnPar
 #pragma unroll
                 for (int j = 0; j < 16; ++j) mx = fmaxf(mx, __uint_as_float(r[h][j]));
         }
-        stat[half * kTile + trow_i] = mx;
-        named_barrier_sync(1 + quarter, 64);
-        mx = fmaxf(mx, stat[(half ^ 1) * kTile + trow_i]);
-        named_barrier_sync(1 + quarter, 64);             // both have read: the slots are free for the row sums
+        if (!idle) {                                     // (both warps of a quarter skip together: the barrier is theirs alone)
+            stat[half * kTile + trow_i] = mx;
+            named_barrier_sync(1 + quarter, 64);
+            mx = fmaxf(mx, stat[(half ^ 1) * kTile + trow_i]);
+            named_barrier_sync(1 + quarter, 64);         // both have read: the slots are free for the row sums
+        }
         if (t == 0) COTR_TS(5);
         const float kLog2e = 1.4426950408889634f;
         const float mxs = mx * kLog2e;
@@ -209,6 +218,11 @@ __global__ void __launch_bounds__(kThreads, 1) attention_tc_kernel(const AttnPar
 #pragma unroll 1
         for (int c = 0; c < kChunks; ++c) {
             const int buf = c & 1;
+            if (idle) {                                  // keep the barrier protocol, skip the work
+                if (c >= 2) mbar_wait(&p_empty[buf], (uint32_t)((c >> 1) - 1) & 1u);
+                mbar_arrive(&p_full[buf]);
+                continue;
+            }
             uint32_t r[2][16];
             __syncwarp();
 #pragma unroll
@@ -242,17 +256,19 @@ __global__ void __launch_bounds__(kThreads, 1) attention_tc_kernel(const AttnPar
             mbar_arrive(&p_full[buf]);
             if (t == 0) COTR_TS(6 + c);
         }
-        stat[half * kTile + trow_i] = sum;
-        named_barrier_sync(1 + quarter, 64);
-        sum += stat[(half ^ 1) * kTile + trow_i];
+        if (!idle) {
+            stat[half * kTile + trow_i] = sum;
+            named_barrier_sync(1 + quarter, 64);
+            sum += stat[(half ^ 1) * kTile + trow_i];
+        }
 
         // ---- O / sum -> global (split16): this thread's 16 of the 32 head-dim columns ------------------------
         mbar_wait(o_full, 0);
         tcgen05_fence_after();
         if (t == 0) COTR_TS(14);
-        const float inv = 1.f / sum;
-        const size_t ooff = grow * p.ldo + head * kHeadDim + half * 16;
-        {
+        if (!idle) {
+            const float inv = 1.f / sum;
+            const size_t ooff = grow * p.ldo + head * kHeadDim + half * 16;
             const uint32_t orow = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)(half * 16);
             uint32_t r0[16], r1[16], r2[16], r3[16];
             __syncwarp();
@@ -345,16 +361,21 @@ __global__ void __launch_bounds__(kThreads, 1) attention_tc_kernel(const AttnPar
 
 int launch_attention_tc(const AttnParams& p, cudaStream_t s) {
     if (p.nq <= 0 || p.npairs <= 0) return 0;
-    if (p.nq < 32) return launch_attention_simt(p, s);   // a 128-row MMA tile would be > 75% padding
+    // a 128-row MMA tile would be > 75% padding: by default such launches run on the SIMT kernel; a scheduling count
+    // of 32 or more (batch-invariant mode, the path-2 test hook) keeps them on the tensor cores
+    if ((p.nq_sched > 0 ? p.nq_sched : p.nq) < 32) return launch_attention_simt(p, s);
+    const bool skip_idle = p.nq < 32;
     static unsigned long long configured = 0;      // bit per device
     if (first_use_on_device(&configured)) {
-        COTR_CHECK_CUDA(cudaFuncSetAttribute(attention_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes));
+        COTR_CHECK_CUDA(cudaFuncSetAttribute(attention_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes));
+        COTR_CHECK_CUDA(cudaFuncSetAttribute(attention_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemBytes));
     }
     COTR_CHECK(p.npairs <= 65535, "attention: too many pairs in one launch (%d)", p.npairs);
     COTR_CHECK((p.ldq & 7) == 0 && (p.ldk & 7) == 0 && (p.ldo & 7) == 0 && (p.vt_pair_stride & 7) == 0,
                "attention_tc: leading dimensions must be multiples of 8 elements");
     dim3 grid((p.nq + kTile - 1) / kTile, kHeads, p.npairs);
-    COTR_CHECK_CUDA(launch_kernel(attention_tc_kernel, grid, dim3(kThreads), kSmemBytes, s, p, next_trace_block()));
+    COTR_CHECK_CUDA(launch_kernel(skip_idle ? attention_tc_kernel<true> : attention_tc_kernel<false>, grid, dim3(kThreads), kSmemBytes, s, p,
+                                  next_trace_block()));
     return 0;
 }
 

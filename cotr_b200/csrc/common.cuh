@@ -284,6 +284,10 @@ struct GemmParams {
     Split16 vt;
     int n_vt;
     unsigned char* kv_img;
+    // Scheduling row count (host side only, never read by a kernel): tile width and split-K are chosen as if the launch
+    // had M_sched rows; 0 = M.  The batch-invariant mode sets it to the row count of the same call site at the
+    // headline shape, so a row's summation order does not depend on how many other rows share the launch.
+    int M_sched;
 };
 
 // softmax(q k^T) v per head; q already carries the head_dim^-0.5 scale.
@@ -301,6 +305,9 @@ struct AttnParams {
     int npairs;
     int pair0;
     LaunchSync sync;             // dataflow dependencies (all zero: hardware griddepcontrol.wait)
+    // Scheduling query count (host side only): launch_attention_tc hands launches with nq_sched < 32 to the SIMT kernel;
+    // 0 = nq.  The batch-invariant mode sets it to the headline's count, so every nq >= 1 runs on the tensor cores.
+    int nq_sched;
 };
 
 int launch_gemm_simt(const GemmParams& p, cudaStream_t s);

@@ -738,10 +738,13 @@ int launch_one(const GemmParams& p, cudaStream_t s) {
     dim3 grid((p.M + BM - 1) / BM, (p.N + BN - 1) / BN);
     // Split-K over a thread-block cluster for long reductions on under-filled grids (the K loop is the serial part of
     // these latency-bound launches): 4 or 2 CTAs per output tile, each >= 4 chunks, at most ~one wave of CTAs.
+    // The grid fill is that of the scheduling row count (GemmParams::M_sched): a larger launch may run split-K over
+    // several waves, so that its rows are summed in the same order as at the scheduling size.
     int ksplit = 1;
     if constexpr (!LN && BN <= 64 && MODE != LD_STEM4) {
         const int kc = (p.K + BK - 1) / BK;
-        const long long ctas = (long long)grid.x * grid.y;
+        const int m_sched = p.M_sched > 0 ? p.M_sched : p.M;
+        const long long ctas = (long long)((m_sched + BM - 1) / BM) * grid.y;
         if (!(g_tc_variant & 512) && kc >= (16 >> ((g_tc_variant >> 14) & 3))) {     // bring-up knob: bits 14-15
             if (C::kMaxSplit >= 4 && kc % 4 == 0 && ctas * 4 <= 160) ksplit = 4;
             else if (C::kMaxSplit >= 2 && kc % 2 == 0 && ctas * 2 <= 160) ksplit = 2;
@@ -876,8 +879,9 @@ int launch_gemm_tc(const GemmParams& p, cudaStream_t s, GemmLaunchInfo* info) {
     }
     // Tile width: at small batch most GEMMs of this network have a handful of 128-row tiles, so the widest tile
     // that still yields ~100 CTAs (148 SMs) wins; the narrow tiles trade tensor efficiency for parallelism and a
-    // shorter per-CTA epilogue (the critical path of these latency-bound launches).
-    const long long mt = (p.M + BM - 1) / BM;
+    // shorter per-CTA epilogue (the critical path of these latency-bound launches).  The tile width sets the number
+    // of TMEM accumulators and so the summation order: it is chosen from the scheduling row count (M_sched).
+    const long long mt = ((p.M_sched > 0 ? p.M_sched : p.M) + BM - 1) / BM;
     // bring-up knobs (cotr_debug_set_variant): bits 10-11 / 12-13 move the CTA-count thresholds of the 64 / 128 tiles
     static const long long kThr[4] = {96, 48, 64, 148};
     static const long long kThrWide[4] = {96, 48, 1 << 30, 148};

@@ -108,6 +108,7 @@ struct cotr_context {
     cotr::Split16 vt = cotr::kNoSplit;   // [max_pairs][6][256][512]  (value projections stored transposed)
     unsigned char* img = nullptr;        // [max_pairs][6][8 heads] attention operand images (common.cuh kAttnHeadImgBytes)
     bool holds_img = false;              // what the last encode wrote: images (tensor-core path) or k / vt (fp32 SIMT path)
+    bool batch_invariant = false;        // the schedule policy the last encode ran under (cotr_set_batch_invariant)
     int max_pairs = 0;
     int pairs = 0;                       // pairs encoded by the last cotr_encode_context
 };
@@ -115,6 +116,7 @@ struct cotr_context {
 struct cotr_model {
     int device = 0;
     int gemm_path = 0;          // 0 = tcgen05, 1 = fp32 SIMT
+    bool batch_invariant = false;   // cotr_set_batch_invariant: every launch scheduled as at the headline shape
     int launches = 0;
     std::vector<void*> allocs;
     cotr::DevConv stem;
@@ -322,7 +324,23 @@ struct Run {
     cotr_model* m;
     cudaStream_t s;
     SyncPlan* sp = nullptr;
+    // batch-invariant schedule (tensor-core path): a launch of M rows is scheduled as if it had sched_rows rows (decoder)
+    // or M / sched_pairs rows (encoder of sched_pairs pairs, i.e. one pair's rows); both 0 = as M rows
+    int sched_pairs = 0;
+    int sched_rows = 0;
 };
+
+// The batch-invariant mode schedules every launch as the same call site at the headline shape (B = 1, Q = 1024): the
+// backbone and encoder as for one pair, the decoder, query projection and head as for 1024 query rows.
+constexpr int kHeadlineQueries = 1024;
+inline bool invariant_schedule(const cotr_model* m) { return m->batch_invariant && m->gemm_path == 0; }
+
+// Row count every schedule decision of a launch with M rows reads (tile width, split-K, LayerNorm placement).
+inline int sched_rows(const Run& r, int M) {
+    if (r.sched_rows > 0) return r.sched_rows;
+    if (r.sched_pairs > 0) return M / r.sched_pairs;
+    return M;
+}
 
 // mode: what this launch would like to wait for (degraded to DEP_ALL when the producer's row tiling does not match);
 // rows: size of this launch's row space; returns the LaunchSync with the dependency part and the signal block filled.
@@ -403,6 +421,7 @@ int launch_tc(const Run& r, GemmParams& p, int dep_mode = DEP_ALL) {
     // only the row-major operand kernels exist in a dataflow-capable form (gemm_tc.cu, DLN instantiations): convolutions
     // keep the hardware wait and announce nothing, so their successor falls back to the hardware wait as well
     const bool flow_ok = (p.a_mode == A_ROWMAJOR || p.a_mode == A_TOKENS) && (p.K & 7) == 0 && (p.lda & 7) == 0;
+    p.M_sched = sched_rows(r, p.M);
     if (flow_ok) p.sync = plan_dep(r, dep_mode, p.M);
     else if (r.sp) r.sp->prev = nullptr;
     p.sync.sig_tiles = p.sync.sig ? sync_tiles_for(p.M) : 0;
@@ -420,7 +439,9 @@ int run_gemm(const Run& r, GemmParams p, float* ln_scratch, int dep_mode = DEP_A
         // The fused LayerNorm epilogue needs the whole 256-wide row in one CTA (128 x 256 tile): with few rows that is
         // a handful of CTAs doing a long serial epilogue while the other SMs idle.  Below ~64 row tiles the GEMM runs
         // with narrow tiles across many SMs and LayerNorm follows as its own (in-place, one warp per row) kernel.
-        const bool defuse = p.ln_gamma != nullptr && (p.M + 127) / 128 < 64;
+        // The batch-invariant schedule decides from its scheduling row count (<= 1024 rows: always separate).
+        p.M_sched = sched_rows(r, p.M);
+        const bool defuse = p.ln_gamma != nullptr && (p.M_sched + 127) / 128 < 64;
         const float* g = p.ln_gamma;
         const float* b = p.ln_beta;
         if (defuse) { p.ln_gamma = nullptr; p.ln_beta = nullptr; }
@@ -506,9 +527,12 @@ int run_conv(const Run& r, const DevConv& c, int n_img, CSplit16 in, int H, int 
 int run_attention(const Run& r, AttnParams p, int dep_mode = DEP_ALL, int span = 0) {
     // recorded as M = query rows, N = 512 keys, K = 32 x 8 heads
     const int rows = p.nq * p.npairs;
-    LaunchScope scope(r, r.m->gemm_path == 0 ? K_ATTN_TC : K_ATTN_SIMT, rows, kTokens, kDModel);
+    if (r.sched_rows > 0) p.nq_sched = r.sched_rows;       // batch-invariant decoder: tcgen05 for every nq >= 1
+    // launch_attention_tc hands launches with fewer than 32 (scheduling) query rows to the SIMT kernel
+    const bool simt = r.m->gemm_path != 0 || (p.nq_sched > 0 ? p.nq_sched : p.nq) < 32;
+    LaunchScope scope(r, simt ? K_ATTN_SIMT : K_ATTN_TC, rows, kTokens, kDModel);
     if (r.m->gemm_path != 0) return launch_attention_simt(p, r.s);
-    if (p.nq < 32) {                          // launch_attention_tc hands these to the SIMT kernel: hardware wait, no announcements
+    if (simt || p.nq < 32) {                  // SIMT, or a partial tile: hardware wait, no announcements
         if (r.sp) r.sp->prev = nullptr;
         return launch_attention_tc(p, r.s);
     }
@@ -673,6 +697,7 @@ int encode_impl(cotr_model* m, const float* img, int B, cotr_context* ctx, cudaS
     plan.cap_blocks = kSyncEncodeBlocks;
     if (plan.on) COTR_CHECK_CUDA(cudaMemsetAsync(w.sync_ctr, 0, (size_t)kSyncEncodeBlocks * kSyncBlockInts * sizeof(int), s));
     Run r{m, s, &plan};
+    if (invariant_schedule(m)) r.sched_pairs = B;
     const int n_img = 2 * B;
     const CSplit16 none{nullptr, nullptr};
 
@@ -727,7 +752,7 @@ int encode_impl(cotr_model* m, const float* img, int B, cotr_context* ctx, cudaS
     // transformer.py:143-159 x6 (post-LN).  q = k = x + pos is folded into the constant add_qkv matrix.
     // q | k land row-major in qk [T][512]; v lands transposed in vt [pair][256][512] (what P V needs as its B operand).
     Split16 xin = w.src;      // layer input
-    if (deferred_ln_enabled(m, T)) {
+    if (deferred_ln_enabled(m, sched_rows(r, T))) {
         // Tensor-core path: no LayerNorm kernel and no LayerNorm epilogue.  A LayerNorm output is never stored; its
         // producer writes the pre-norm rows (xa: x + attention, xb: x1 + FFN) and every consumer applies the norm on
         // the fly (GemmParams::a_ln_cs for GEMM inputs, res_ln_part for residual operands) from the partial row
@@ -787,6 +812,7 @@ int encode_impl(cotr_model* m, const float* img, int B, cotr_context* ctx, cudaS
         }
         ctx->pairs = B;
         ctx->holds_img = true;
+        ctx->batch_invariant = m->batch_invariant;
         m->last_pairs = B;
         return 0;
     }
@@ -841,6 +867,7 @@ int encode_impl(cotr_model* m, const float* img, int B, cotr_context* ctx, cudaS
     }
     ctx->pairs = B;
     ctx->holds_img = tc;
+    ctx->batch_invariant = m->batch_invariant;
     m->last_pairs = B;
     return 0;
 }
@@ -855,6 +882,7 @@ int decode_chunk(cotr_model* m, const cotr_context* ctx, const float* queries, f
     plan.base = w.sync_ctr + (size_t)(kSyncEncodeBlocks + chunk_index * kSyncChunkBlocks) * kSyncBlockInts;
     plan.cap_blocks = kSyncChunkBlocks;
     Run r{m, s, &plan};
+    if (invariant_schedule(m)) r.sched_rows = kHeadlineQueries;
     const int R = npairs * nq;
     const CSplit16 none{nullptr, nullptr};
     // cotr_model.py:34-35 query_proj (lin_sine, depth 64)
@@ -869,7 +897,7 @@ int decode_chunk(cotr_model* m, const cotr_context* ctx, const float* queries, f
     // all 6 layers is one GEMM.
     if (run_linear(r, m->qpos_all, R, cs(w.qpos), kDModel, w.qp, kQpCols, false, none, 0, nullptr, nullptr, nullptr, DEP_TILE)) return 1;
 
-    if (deferred_ln_enabled(m, R)) {
+    if (deferred_ln_enabled(m, sched_rows(r, R))) {
         // Tensor-core path with deferred LayerNorms (see encode_impl): w.t = t + attention (norm2 deferred),
         // w.t2 = t1 + FFN (norm3 deferred); dec_st_a = partial row statistics of w.t (norm2), dec_st_b of w.t2 (norm3).
         for (int l = 0; l < kDecLayers; ++l) {
@@ -953,6 +981,9 @@ int decode_impl(cotr_model* m, const cotr_context* ctx, const float* queries, in
     COTR_CHECK(Q >= 0, "cotr_decode: negative Q");
     COTR_CHECK(ctx->holds_img == (m->gemm_path == 0), "cotr_decode: the context was encoded under the other matrix-multiply path "
                "(cotr_set_gemm_path): re-encode it");
+    COTR_CHECK(ctx->batch_invariant == m->batch_invariant, "cotr_decode: the context was encoded with batch-invariant mode %s and the "
+               "model now has it %s (cotr_set_batch_invariant): re-encode it", ctx->batch_invariant ? "on" : "off",
+               m->batch_invariant ? "on" : "off");
     if (Q == 0) return 0;
     COTR_CHECK_CUDA(cudaSetDevice(m->device));
     const long long total = (long long)B * Q;
@@ -1523,6 +1554,19 @@ int cotr_set_gemm_path(cotr_model* m, int path) {
     return 0;
 }
 
+int cotr_set_batch_invariant(cotr_model* m, int enabled) {
+    COTR_CHECK(m != nullptr, "cotr_set_batch_invariant: null model");
+    const bool on = enabled != 0;
+    if (m->batch_invariant != on) {      // a graph captured under one policy must never replay under the other
+        cudaSetDevice(m->device);
+        cudaDeviceSynchronize();
+        drop_graphs(m);
+        m->shapes_seen.clear();
+    }
+    m->batch_invariant = on;
+    return 0;
+}
+
 void cotr_debug_set_variant(int variant) { g_tc_variant = variant; g_use_pdl = (variant & 256) ? 0 : 1; }
 void cotr_debug_set_timestamps(void* dev_buffer) {
     g_tc_timestamps = reinterpret_cast<long long*>(dev_buffer);
@@ -1674,6 +1718,7 @@ int cotr_test_gemm(const cotr_test_gemm_desc* d, const float* A_dev, const float
 int cotr_test_attention(int path, const float* q_dev, const float* k_dev, const float* v_dev, float* out_dev,
                         int nq, int npairs) {
     COTR_CHECK(q_dev && k_dev && v_dev && out_dev, "cotr_test_attention: null argument");
+    COTR_CHECK(path >= 0 && path <= 2, "cotr_test_attention: path must be 0, 1 or 2");
     TmpSplit q16, k16, vt16, o16;
     const size_t qn = (size_t)npairs * nq * kDModel, kn = (size_t)npairs * kTokens * kDModel;
     if (q16.from_f32(q_dev, qn) || k16.from_f32(k_dev, kn) || vt16.empty(kn) || o16.empty(qn)) return 1;
@@ -1700,7 +1745,8 @@ int cotr_test_attention(int path, const float* q_dev, const float* k_dev, const 
     a.q = cs(q16.t); a.ldq = kDModel; a.k = cs(k16.t); a.ldk = kDModel;
     a.vt = cs(vt16.t); a.vt_pair_stride = kVtLayer;
     a.out = o16.t; a.ldo = kDModel; a.nq = nq; a.npairs = npairs; a.pair0 = 0;
-    int rc = path == 0 ? launch_attention_tc(a, 0) : launch_attention_simt(a, 0);
+    if (path == 2) a.nq_sched = kHeadlineQueries;      // tcgen05 whatever nq (as in the batch-invariant schedule)
+    int rc = path == 1 ? launch_attention_simt(a, 0) : launch_attention_tc(a, 0);
     if (!rc) rc = launch_split16_to_f32(cs(o16.t), out_dev, qn, 0);
     cudaError_t e = cudaDeviceSynchronize();
     if (rc) return rc;

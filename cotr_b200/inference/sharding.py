@@ -13,7 +13,10 @@ Two entry points:
     (SPMD): every rank executes the same engine code with the same seeds, every model call is split over the ranks
     (contexts contiguously; the single-context dense pass of cotr_flow over its 131 072 queries) and all-gathered, so
     every rank sees identical predictions and takes identical decisions.  Task state therefore needs no broadcast,
-    and rank 0's return value is the job's result.
+    and rank 0's return value is the job's result.  That holds bit for bit only if a rank's predictions for a pair or a
+    query do not depend on which other pairs / queries share its call: with the wrapped model in batch-invariant mode
+    (`COTR.batch_invariant`) the job's result is the same on any number of ranks.  The ranks must agree on the mode,
+    which `ShardedCOTR` checks when it is constructed.
 """
 import numpy as np
 import torch
@@ -205,6 +208,14 @@ class ShardedCOTR(nn.Module):
         super().__init__()
         self.model = model
         self.group = group
+        if _active(group):
+            # collective: a rank whose model runs another schedule would make other decisions and silently diverge
+            mine = bool(getattr(model, 'batch_invariant', False))
+            modes = [None] * dist.get_world_size(group)
+            dist.all_gather_object(modes, mine, group=group)
+            if len(set(modes)) != 1:
+                raise RuntimeError(f"ShardedCOTR: the ranks' models disagree on batch_invariant (by rank: {modes}); "
+                                   "set the same mode on every rank")
 
     @property
     def supports_device_preprocess(self):

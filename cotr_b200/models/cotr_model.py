@@ -8,6 +8,11 @@ Reference contract (COTR/models/cotr_model.py:17-51):
   * `forward(samples, queries) -> {'pred_corrs': (B,Q,2)}` on the module's device; samples is a (B,3,256,512) tensor,
     a list of (3,256,512) tensors or a NestedTensor; the canvas size is asserted like backbone.py:80.
 
+`batch_invariant` (off by default; `args.batch_invariant` or `set_batch_invariant`) makes every pair and query come out
+bit-identical whatever else shares the call: batch size, query count, decode chunking, entry point, rank count
+(cotr_set_batch_invariant in include/cotr_b200.h).  It is a property of the handle, not a parameter: the state_dict is
+the same in both modes.
+
 The arithmetic is NOT done by torch: forward hands device pointers to libcotr_b200.so (include/cotr_b200.h).
 There is no CPU path; calling forward without a CUDA device or without the built library raises.
 Unlike the reference constructor (backbone.py:106 `pretrained=True`) nothing is downloaded.
@@ -170,6 +175,7 @@ class COTR(nn.Module):
         self.backbone = backbone
         self._native = None
         self._ctx_cache = {}
+        self._batch_invariant = bool(getattr(args, "batch_invariant", False)) if args is not None else False
 
     # ---- native handle management ---------------------------------------------------------------------
     def _invalidate(self):
@@ -199,8 +205,29 @@ class COTR(nn.Module):
                 raise RuntimeError("cotr_b200.COTR runs only on a CUDA device (sm_100a): call model.cuda() first; "
                                    "there is no CPU fallback")
             idx = dev.index if dev.index is not None else torch.cuda.current_device()
-            self._native = capi.NativeModel(self.state_dict(), idx)
+            nat = capi.NativeModel(self.state_dict(), idx)
+            if self._batch_invariant:
+                nat.set_batch_invariant(True)
+            self._native = nat
         return self._native
+
+    @property
+    def batch_invariant(self):
+        """True: predictions are bit-identical for any batch size, query count, chunking, entry point or rank count."""
+        return self._batch_invariant
+
+    def set_batch_invariant(self, enabled):
+        """Switch the batch-invariant mode.  Cached encode_context(reuse=True) contexts are closed (a context is only
+        valid under the mode it was encoded in); the packed weights are kept."""
+        enabled = bool(enabled)
+        if enabled == self._batch_invariant:
+            return
+        self._batch_invariant = enabled
+        for ctx in self._ctx_cache.values():
+            ctx.close()
+        self._ctx_cache = {}
+        if self._native is not None:
+            self._native.set_batch_invariant(enabled)
 
     # ---- reference API --------------------------------------------------------------------------------
     def _canvas(self, samples):

@@ -171,8 +171,8 @@ int cotr_last_launch_count(const cotr_model* m);
 /* Per-launch profiler.  Between cotr_profile_begin and cotr_profile_end every kernel the library launches is bracketed
  * by two CUDA events recorded on the launching stream.  cotr_profile_end synchronises the device, fills `out` with
  * one record per launch in launch order and returns -(count + 1) on success (so 0 records -> -1), > 0 on failure.
- * kernel ids: 0 gemm_tc (tcgen05), 1 gemm_simt, 2 attention_tc, 3 attention_simt, 4 layernorm, 5 maxpool,
- * 6 query_encode, 7 stem_canvas.  For GEMMs M,N,K are the problem size; for attention M = query rows, N = 512, K = 256. */
+ * kernel ids: 0 gemm_tc (tcgen05), 1 gemm_simt, 2 attention_tc, 3 attention_simt (the fp32 path, and the default
+ * schedule's attention of launches with fewer than 32 queries per pair), 4 layernorm, 5 maxpool, 6 query_encode, 7 stem_canvas.  For GEMMs M,N,K are the problem size; for attention M = query rows, N = 512, K = 256. */
 typedef struct cotr_launch_record {
     int32_t kernel;
     int32_t M, N, K;
@@ -190,6 +190,26 @@ int64_t cotr_debug_read(cotr_model* m, const char* name, float* out_host, int64_
 /* Select the matrix-multiply path: 0 = tcgen05 tensor-core kernels (default), 1 = fp32 SIMT kernels
  * (debug / numerical cross-check only). */
 int cotr_set_gemm_path(cotr_model* m, int path);
+
+/* Batch-invariant inference mode (0 = off, the default).  By default each launch picks its schedule - GEMM tile width,
+ * split-K, fused or separate LayerNorm, deferred LayerNorm, tensor-core or SIMT attention - from its own row count, so
+ * a pair's predictions move in the last bits with the batch size, the query count and the decode chunking.  With the
+ * mode on, every pair and every query is computed by the kernel sequence of the headline forward (B = 1, Q = 1024)
+ * whatever B, Q, chunking or entry point the call has: the backbone and encoder are scheduled as for one pair, the
+ * decoder, query projection and head as for 1024 query rows, LayerNorms run as separate launches and attention runs on
+ * the tensor cores for any query count.  Consequences, all bitwise:
+ *   - pair p alone gives the same predictions as pair p inside any batch;
+ *   - a query gives the same prediction alone or among any others, at any position, across decode chunks and next to
+ *     zero-padded queries;
+ *   - cotr_forward, cotr_encode_context + any split of the queries over cotr_decode calls, cotr_forward_host, graph
+ *     replay and eager execution agree;
+ *   - at B = 1, Q = 1024 both modes launch the same kernels and produce the same bits.
+ * Larger calls may be slower in this mode (narrow split-K tiles on big grids, separate LayerNorm launches).  The flag
+ * belongs to the model handle.  Toggling it synchronises the device and drops captured graphs, like
+ * cotr_set_gemm_path.  A context records the mode it was encoded under; cotr_decode refuses a context encoded under
+ * the other mode.  The fp32 SIMT path (cotr_set_gemm_path 1) ignores the flag.  Bring-up switches of
+ * cotr_debug_set_variant apply to every launch alike, so the guarantees hold under any fixed variant value. */
+int cotr_set_batch_invariant(cotr_model* m, int enabled);
 
 /* ---- kernel-level test hooks (used by tests/ only) ------------------------------------------------------ */
 typedef struct cotr_test_gemm_desc {
@@ -213,7 +233,9 @@ typedef struct cotr_test_gemm_desc {
 int cotr_test_gemm(const cotr_test_gemm_desc* d, const float* A_dev, const float* w_host, const float* bias_dev,
                    const float* addmat_dev, const float* residual_dev, const float* ln_gamma_dev,
                    const float* ln_beta_dev, float* out_dev, float* part_out_dev /* [M][16][2] or NULL */);
-/* out[(p*nq+i), h*32+d] = softmax(q k^T) v per head; q (npairs*nq,256), k/v (npairs*512,256), all DEVICE, ld 256. */
+/* out[(p*nq+i), h*32+d] = softmax(q k^T) v per head; q (npairs*nq,256), k/v (npairs*512,256), all DEVICE, ld 256.
+ * path: 0 = tcgen05 as the default schedule runs it (nq < 32 goes to the SIMT kernel), 1 = SIMT, 2 = tcgen05 for any
+ * nq >= 1 (the batch-invariant schedule). */
 int cotr_test_attention(int path, const float* q_dev, const float* k_dev, const float* v_dev, float* out_dev,
                         int nq, int npairs);
 /* bring-up / A-B switches (0 = production): bit 8 (256) disables programmatic dependent launch, bit 9 (512) disables

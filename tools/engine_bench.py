@@ -64,9 +64,10 @@ def forced_cycle_consistency(engine, img_a, img_b, queries_a, max_corrs):
 
 
 def compare_runs(single, sharded):
-    """Two runs of the same job whose model calls were batched differently (1 rank vs N ranks).  The network's answers
-    agree to ~1e-6 of the image, not bit for bit (the GEMM tile shapes follow the rows per launch), so the 2048 survivors
-    of the cycle-error ranking may differ near the cut: report the overlap and the differences on the common points."""
+    """Two runs of the same job whose model calls were batched differently (1 rank vs N ranks).  In the default mode the
+    network's answers agree to ~1e-6 of the image, not bit for bit (the GEMM tile shapes follow the rows per launch), so
+    the 2048 survivors of the cycle-error ranking may differ near the cut: report the overlap and the differences on the
+    common points.  In batch-invariant mode (COTR.set_batch_invariant) the two runs must be identical."""
     same_order = single.shape == sharded.shape and bool(np.array_equal(single[:, :2], sharded[:, :2]))
     a = {tuple(r[:2]): r[2:] for r in single}
     common = [(a[tuple(r[:2])], r[2:]) for r in sharded if tuple(r[:2]) in a]
